@@ -9,7 +9,7 @@ the reference's relative paths assume (`pretrained_models/...`, `models/sean_cod
     from hair_swap import HairFast, get_parser    # the reference's own file, unchanged
 
 One process = one mode (the reference's modules are cached in sys.modules).  Nothing here is product code: it is the
-harness of tests/test_gpu_swap.py, of `bench.py`'s full-swap / reference legs and of tools/dryrun_swap_cpu.py.
+harness of baseline/run_swap.py, of `bench.py`'s full-swap / reference legs and of tools/dryrun_swap_cpu.py.
 """
 from __future__ import annotations
 

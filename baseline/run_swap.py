@@ -11,7 +11,7 @@ checkpoints come from baseline/synth_checkpoints.py, `swap(..., seed=3407)` is t
 The result file holds the final image of every repetition, the Embedding-stage latents of the last one and the wall /
 CUDA-event timings: whole swap, and the share spent inside the hot-path modules (generator, e4e, FS encoder,
 PostProcess conv stack, BiSeNet) measured with forward hooks -- the hot-path / out-of-scope split of SURVEY 8d.
-Harness (tests/test_gpu_swap.py, bench.py's full-swap leg); not product code.
+Harness (run by hand; bench.py's full-swap leg); not product code.
 """
 from __future__ import annotations
 

@@ -183,38 +183,44 @@ def run_ours(args, rank, world, local_rank):
     host_out = torch.empty(T, 3, 1024, 1024).pin_memory()
     launches = [0]
 
-    def compute(inp, skip_fse_recon=False, full_seg=False):
-        """The hot path of T triples through the public module API (what swap()'s stages call)."""
+    def compute(inp, skip_fse_recon=False, full_seg=False, outs=None):
+        """The hot path of T triples through the public module API (what swap()'s stages call).  `outs`, if given,
+        receives every network output of the step by name."""
+        def keep(name, out):
+            if outs is not None:
+                outs[name] = out
+            return out
         img, lats, lins, calls = inp["img"], inp["lat"], inp["lin"], inp["calls"]
         n0 = lib.hf_total_launch_count() + graphs.stats()["replayed_kernels"]   # eager launches + kernels inside replayed graphs
-        for net, x in ((e4e, img[0]), (e4e, img[1]), (fse, img[2])):   # Embedding.py:71,74 / :51
-            net(x)
+        for name, net, x in (("e4e_a", e4e, img[0]), ("e4e_b", e4e, img[1]), ("fse", fse, img[2])):   # Embedding.py:71,74 / :51
+            keep(name, net(x))
         final = None
         for i, (s, e, b, r) in enumerate(calls):
             if i == 0 and skip_fse_recon:              # opt-in 8f-2 fast path: same RNG draws, no reconstruction
                 gen.consume_noise(b)
                 continue
-            out = gen([lats[i]], input_is_latent=True, start_layer=s, end_layer=e, layer_in=lins[i])   # random noise
+            out = keep(f"gen{i}_{s}_{e}", gen([lats[i]], input_is_latent=True, start_layer=s, end_layer=e,
+                                              layer_in=lins[i]))                                   # random noise
             if i == len(calls) - 1:
                 final = out[0]
-        _, (f_face,) = pp_enc(img[3])                  # PostProcessModel.forward, models/Encoders.py:120-139
-        _, (f_hair,) = pp_enc(img[4])
-        pp_res(torch.cat((f_face, f_hair), dim=1))
+        _, (f_face,) = keep("pp_enc_face", pp_enc(img[3]))   # PostProcessModel.forward, models/Encoders.py:120-139
+        _, (f_hair,) = keep("pp_enc_hair", pp_enc(img[4]))
+        keep("pp_res", pp_res(torch.cat((f_face, f_hair), dim=1)))
         # get_segmentation x3 at 512^2 and twice at 1024^2 (models/Net.py:108-115).  Under install()'s defaults the
         # reference's FaceParsing_tensor.parsing_img runs the label-only path (parsing_fast.py: bit-identical labels,
         # aux heads + full-resolution logits not materialised); `full_seg=True` = the module's three-logit forward
         parse = seg if full_seg else seg.parse_labels
-        parse(img[5])
-        parse(img[6]); parse(img[6])
+        keep("seg_512", parse(img[5]))
+        keep("seg_1024_a", parse(img[6])); keep("seg_1024_b", parse(img[6]))
         launches[0] += lib.hf_total_launch_count() + graphs.stats()["replayed_kernels"] - n0
         return final
 
-    def step():
-        return compute(devin)
+    def step(outs=None):
+        return compute(devin, outs=outs)
 
     flush = torch.empty(256 << 20, dtype=torch.uint8, device=dev)     # > 126 MB L2
 
-    def timed(steps: int, warmup: int):
+    def timed(steps: int, warmup: int, outs=None):
         for _ in range(warmup):
             step()
         torch.cuda.synchronize()
@@ -223,11 +229,11 @@ def run_ours(args, rank, world, local_rank):
         torch.cuda.synchronize()
         launches[0] = 0
         total_ms = 0.0
-        for _ in range(steps):
+        for k in range(steps):
             flush.fill_(1)                                             # L2 flush between timed iterations
             e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
             e0.record()
-            step()
+            step(outs if k == steps - 1 else None)
             e1.record()
             e1.synchronize()
             total_ms += e0.elapsed_time(e1)
@@ -305,7 +311,11 @@ def run_ours(args, rank, world, local_rank):
         step()                                        # also gives nvidia-smi time to start sampling
     torch.cuda.synchronize()
     first = sampler.mark()
-    ms, n_launch = timed(args.steps, args.warmup)
+    outs = {} if args.dump_outputs and rank == 0 else None
+    ms, n_launch = timed(args.steps, args.warmup, outs)
+    if outs is not None:
+        dump_outputs(outs, args.dump_outputs)
+        del outs
     ms_e2e = timed_e2e(args.steps, max(3, args.warmup // 2))
     clocks = sampler.stop(first) if rank == 0 else None
 
@@ -426,6 +436,38 @@ def run_ours(args, rank, world, local_rank):
     h2d = sum(t.numel() * 4 for t in host["lat"]) + sum(t.numel() * 4 for t in host["lin"] if t is not None) \
         + sum(t.numel() * 4 for t in host["img"])
     return ms, ms_e2e, n_launch, clocks, extra, h2d
+
+
+DUMP_BYTES = 64 << 20
+
+
+def dump_outputs(outs, path):
+    """Write every tensor in `outs` (name -> tensor or nested tuple / list; None entries skipped) as
+    path/<name>[.<index>...].npy in float32.  A tensor larger than its even share of DUMP_BYTES is written as a fixed
+    sample of its flattened elements (indices drawn from a generator seeded by the name, sorted), so that two builds
+    run with the same arguments write files that compare element for element."""
+    import zlib
+    import numpy as np
+    import torch
+    leaves = []
+
+    def walk(name, v):
+        if torch.is_tensor(v):
+            leaves.append((name, v))
+        elif isinstance(v, (list, tuple)):
+            for j, u in enumerate(v):
+                walk(f"{name}.{j}", u)
+    for name, v in outs.items():
+        walk(name, v)
+    share = (DUMP_BYTES - 4096 * len(leaves)) // (4 * len(leaves))      # 4096: room for each .npy header
+    os.makedirs(path, exist_ok=True)
+    for name, t in leaves:
+        t = t.detach()
+        if t.numel() > share:
+            g = torch.Generator().manual_seed(zlib.crc32(name.encode()))
+            idx = torch.randint(t.numel(), (share,), generator=g).sort().values
+            t = t.reshape(-1)[idx.to(t.device)]
+        np.save(os.path.join(path, name + ".npy"), t.float().cpu().numpy())
 
 
 def _json_tail(stdout: str):
@@ -701,6 +743,9 @@ def main():
     ap.add_argument("--profile-step", action="store_true", help="run one step between cudaProfilerStart/Stop, no JSON")
     ap.add_argument("--no-comparators", action="store_true",
                     help="skip the child-process legs (reference_gpu, full_swap, value_by_dtype)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the network outputs of the last timed step as DIR/<name>.npy (float32, 64 MB in all: "
+                         "larger outputs as a fixed seeded sample); same arguments, same inputs")
     args = ap.parse_args()
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))

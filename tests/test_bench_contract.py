@@ -21,14 +21,10 @@ def _run(*args, timeout=900, env=None):
     return json.loads(lines[0])
 
 
-@pytest.mark.parametrize("arm", ["reference", "port"])
+@pytest.mark.parametrize("arm", ["port"])
 def test_reference_arm_line(arm):
-    """`--impl reference`: the stock reference modules on the host cores when the checkout is staged (kind
-    "reference"), the oracle port otherwise (kind "port"); OMP_NUM_THREADS=1 as torchrun exports it must not shrink
-    the thread count."""
-    from baseline import refenv
-    if arm == "reference" and not refenv.available():
-        pytest.skip("reference checkout not staged")
+    """`--impl reference` without a staged reference checkout: the census on the oracle port (kind "port");
+    OMP_NUM_THREADS=1 as torchrun exports it must not shrink the thread count."""
     d = _run("--impl", "reference", "--steps", "1", "--warmup", "0", env={"HAIRFAST_CPU_ARM": arm,
                                                                           "OMP_NUM_THREADS": "1"})
     assert BASE_KEYS <= set(d) and d["impl"] == "reference"
@@ -40,9 +36,34 @@ def test_reference_arm_line(arm):
     assert "workload" in d["config"] and set(cb["per_call_s"]) >= {"gen_full", "e4e", "seg_1024"}
 
 
+def test_dump_outputs_budget_and_sample(tmp_path):
+    """bench.dump_outputs: nested outputs by name, float32, small arrays whole, large ones as the same seeded sample
+    on every call, 64 MB in all."""
+    import numpy as np
+    import torch
+    sys.path.insert(0, ROOT)
+    import bench
+    outs = {"small": torch.arange(12, dtype=torch.int64).reshape(3, 4),
+            "nested": (torch.randn(40_000_000, generator=torch.Generator().manual_seed(0)), None,
+                       [torch.ones(2, 2, dtype=torch.bfloat16)]),
+            "absent": None}
+    for d in ("a", "b"):
+        bench.dump_outputs(outs, str(tmp_path / d))
+    names = sorted(os.listdir(tmp_path / "a"))
+    assert names == ["nested.0.npy", "nested.2.0.npy", "small.npy"]
+    assert sum(os.path.getsize(tmp_path / "a" / n) for n in names) <= bench.DUMP_BYTES
+    small = np.load(tmp_path / "a" / "small.npy")
+    assert small.dtype == np.float32 and np.array_equal(small, np.arange(12).reshape(3, 4))
+    big = np.load(tmp_path / "a" / "nested.0.npy")
+    assert big.dtype == np.float32 and 0 < big.size < 40_000_000
+    assert np.isin(big, outs["nested"][0].numpy()).all()
+    for n in names:
+        assert np.array_equal(np.load(tmp_path / "a" / n), np.load(tmp_path / "b" / n)), n
+
+
 @pytest.mark.gpu
-def test_our_arm_line():
-    d = _run("--steps", "2", "--warmup", "3", "--triples", "2", "--no-extras")
+def test_our_arm_line(tmp_path):
+    d = _run("--steps", "2", "--warmup", "3", "--triples", "2", "--no-extras", "--dump-outputs", str(tmp_path))
     assert BASE_KEYS <= set(d) and "impl" not in d
     assert d["n_gpus"] == 1 and d["steps"] == 2 and d["warmup"] == 3 and d["scaling"] == "weak"
     assert d["value"] > 0 and abs(d["value"] - 2 / (d["ms_per_step"] * 1e-3)) < 1e-2 * d["value"]
@@ -58,6 +79,9 @@ def test_our_arm_line():
     assert cb["kind"] in ("port", "reference") and cb["cores"] >= 1 and cb["value"] > 0
     assert d["config"]["triples_per_step_per_gpu"] == 2 and "workload" in d["config"]
     assert d["latency_T1"]["latency_ms_per_triple"] > 0
+    dumped = {n: os.path.getsize(tmp_path / n) for n in os.listdir(tmp_path)}
+    assert {"e4e_a.npy", "fse.0.npy", "gen7_5_8.0.npy", "pp_res.npy", "seg_1024_b.npy"} <= set(dumped)
+    assert sum(dumped.values()) <= 64 << 20
 
 
 @pytest.mark.gpu

@@ -8,7 +8,7 @@
 #         baseline/_ref/ext/           the reference's two JIT extensions (op/fused_act.py:10-16,
 #                                      op/upfirdn2d.py:10-16) prebuilt for sm_100a by baseline/build_ref_ext.py so the
 #                                      GPU box does not spend 2.5 min of nvcc per process on them
-# The staged tree is what `bench.py --impl reference`, `bench.py`'s `reference_gpu` leg and tests/test_gpu_swap.py run.
+# The staged tree is what `bench.py --impl reference`, `bench.py`'s `reference_gpu` leg and baseline/run_swap.py run.
 set -euo pipefail
 SRC="${1:-/root/reference}"
 ROOT="$(cd "$(dirname "$0")/.." && pwd)"
